@@ -39,7 +39,7 @@ class B200Inference:
     @staticmethod
     def args_from_train_config(train_config):
         """(scene, [sampling_net, shading_net], threshold, K) read from an initialised reference TrainConfig -- no device
-        needed (tests/test_adapter_config.py runs this against the live reference)."""
+        needed (tests/test_adapter_config.py runs this on the fields of a reference TrainConfig)."""
         f1 = train_config.f_in[1]
         info = train_config.dataset_info
         scene = dict(view_cell_center=list(info.view.view_cell_center), view_cell_size=list(info.view.view_cell_size),

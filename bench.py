@@ -2,6 +2,7 @@
 """bench.py -- frames/s of the AdaNeRF hot path (BASELINE.json metric: frames/sec at 800x800 and rays/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--single-process]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path (rays -> sampling MLP -> threshold / compaction -> posenc -> shading MLP ->
 composite) over one frame of synthetic input: procedurally generated pinhole rays from the view-cell centre, random-init
@@ -20,6 +21,9 @@ checkpoints offline).
           ncclCommInitAll, grouped send / recv gather) instead of one torchrun rank per GPU.
   --impl reference : the reference's CPU path (the oracle port of TrainConfig.inference, torch CPU, all host threads); every
           step is a bounded ray sample of the same frame.
+  --dump-outputs DIR : after the timed steps, the RGB frame of the last timed step -- what the caller of the timed path
+          receives: the frame at N = 1, the gathered frame on the first GPU at N > 1 -- as DIR/rgb.npy, float32 [rays, 3].
+          The inputs are a function of the arguments only, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -31,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark only reads the tree, which may be read-only
 
 WORKLOADS = {
     # BASELINE.json configs[1]: 800x800, thr 0.2, K = 8 (~8 samples/ray with random-init nets: every ray saturates at K)
@@ -51,6 +56,7 @@ for _k in (8, 16):
 FLOP_PER_SAMPLE_MLP1 = 1186816.0   # SURVEY.md 8(d): 2 * 593 408 MAC, unpadded
 FLOP_PER_RAY_MLP0 = 898048.0
 SHADING_KERNEL = "mlp_sh_kernel"
+DUMP_BYTES = 64 << 20
 PAVILLON_NPZ = os.path.join(ROOT, "tests", "golden", "weights_pavillon.npz")
 
 
@@ -163,6 +169,17 @@ def workload_config(name, cfg, n_gpus):
                 scaling=cfg["scaling"], parallelism=par,
                 l2="per-frame working set (packed features + activations I/O, >1 GB) exceeds the 126 MB L2; no explicit flush",
                 mlp0="bf16x3 split precision (fp32-class)", mlp1="bf16 operands, fp32 accumulate")
+
+
+def dump_outputs(out_dir, arrays):
+    """name -> array as <out_dir>/<name>.npy in float32.  An array larger than its share of DUMP_BYTES keeps every s-th
+    row only (the smallest s that fits), the same rows on every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32)
+        stride = -(-a.nbytes // (DUMP_BYTES // len(arrays)))
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[::stride]))
 
 
 # ------------------------------------------------------------------------------------------------- CPU reference arm
@@ -365,6 +382,10 @@ def run_ours(args, cfg, name):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    last = (args.steps - 1) & 1          # buffers of the last timed frame, overwritten by the e2e and profiled renders below
+    last_rgb = None
+    if args.dump_outputs and rank == 0:
+        last_rgb = (frames[last] if world > 1 and gather_mode != "none" else bands[last]).cpu().numpy()
     ms_by_rank = [ms / args.steps]
     if world > 1:
         t = torch.tensor([ms], device="cuda")
@@ -474,6 +495,8 @@ def run_ours(args, cfg, name):
             cpu_baseline=dict(value=cpu["frames_per_s"], unit="frames/s", cores=cpu["cores"], kind="port", sample=cpu["sample"]),
         )
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dict(rgb=last_rgb))
     r.close()
     if world > 1:
         dist.destroy_process_group()
@@ -517,8 +540,9 @@ def run_single_process(args, cfg, name):
     for _ in range(args.steps - 1):
         m.render_camera(pose, rot, W, Hn, thr, K)     # frame f + 1 enqueued before frame f is read
         m.wait_frame()
-    m.wait_frame()
+    frame = m.wait_frame()
     secs = time.perf_counter() - t0
+    last_rgb = frame.cpu().numpy() if args.dump_outputs else None    # the library reuses the frame's buffer
     clocks = sampler.stop()
     render_ms, gather_ms = m.last_times()
     host = torch.empty((W * Hn, 3), dtype=torch.float32).pin_memory().numpy()   # caller-owned page-locked frame buffer
@@ -539,6 +563,8 @@ def run_single_process(args, cfg, name):
                          api="adn_multi_render_camera + adn_multi_wait_frame(host)", finite=bool(np.isfinite(host).all())),
                 clocks=clocks)
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(rgb=last_rgb))
     m.close()
 
 
@@ -551,7 +577,12 @@ def main():
     ap.add_argument("--workload", default="800x800_thr0.2_K8", choices=sorted(WORKLOADS))
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU baseline sample budget")
     ap.add_argument("--single-process", action="store_true", help="drive --gpus devices from one process (multi-GPU C ABI)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm's steps are time-bounded ray samples, not fixed outputs")
     cfg = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, cfg, args.workload)

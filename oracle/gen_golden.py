@@ -2,13 +2,16 @@
 (/root/reference/src, imported through oracle/ref_harness.py) on CPU in the build container.
 
     python oracle/gen_golden.py            # rewrites tests/golden/
+    python oracle/gen_golden.py NAME...    # only the fixtures written by the named functions
 
 The fixtures pin oracle/adanerf_oracle.py (tests/test_oracle_golden.py) and are what the `-m gpu`
 parity tests compare the CUDA path with on the GPU box, where /root/reference does not exist.
 Every file records torch version + thread count (the reference's GEMMs are ATen/oneMKL calls).
 """
+import hashlib
 import json
 import os
+import shutil
 import sys
 
 import numpy as np
@@ -20,7 +23,7 @@ sys.path.insert(0, ROOT)
 
 from oracle import ref_harness as rh          # noqa: E402
 from oracle import adanerf_oracle as orc      # noqa: E402
-from adanerf_b200.onnx_weights import read_onnx_initializers  # noqa: E402
+from adanerf_b200.onnx_weights import read_onnx_initializers, _enc_varint, _field, _fields, _varint  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
 RX = torch.tensor([[1, 0, 0], [0, 0, -1], [0, 1, 0]], dtype=torch.float32)  # camera -z -> world +y
@@ -100,6 +103,126 @@ def stage2_stress():
     save("stage2_stress.npz", **arrays)
 
 
+FRESH_SEEDS = [(11, 8, 0.2), (12, 4, 0.05), (13, 16, 0.3)]
+
+
+def state_dict_digest(sd):
+    """sha256 over the names and fp32 bytes of a state_dict, in its own order."""
+    h = hashlib.sha256()
+    for k, v in sd.items():
+        h.update(k.encode())
+        h.update(np.ascontiguousarray(v.detach().cpu().numpy(), dtype="<f4").tobytes())
+    return h.hexdigest()
+
+
+def fresh_seeds(n_rays=512, n_raw0=64):
+    """The reference initialised from fresh seeds (its own initialisers), then run on a ragged-count variant of those
+    weights.  Stored per case: the digests of the initial weights, the inputs, and the outputs of one inference call
+    (raw0 only for a seeded sample of the rays)."""
+    scene = orc.SCENE_BARBERSHOP
+    dirs_all = torch.from_numpy(orc.generate_ray_directions(800, 800, scene["fov"]).reshape(-1, 3)).float()
+    arrays = dict(meta=meta(case="fresh_seeds", cases=FRESH_SEEDS, scene_params=scene))
+    for seed, K, thr in FRESH_SEEDS:
+        ref = rh.RefRenderer(scene, K=K, thr=thr, seed=seed)
+        sd0 = {k: v.clone() for k, v in ref.models[0].state_dict().items()}
+        sd1 = {k: v.clone() for k, v in ref.models[1].state_dict().items()}
+        tag = f"s{seed}"
+        arrays[tag + "/init_digest"] = np.array([state_dict_digest(sd0), state_dict_digest(sd1)])
+        sd0["layers.7.weight"] *= 0.15                  # ragged sample counts
+        sd0["layers.7.bias"] = sd0["layers.7.bias"] * 0.15 - 0.2
+        ref.load_state_dicts(sd0, sd1)
+        g = torch.Generator().manual_seed(seed)
+        pix = torch.randperm(dirs_all.shape[0], generator=g)[:n_rays]
+        pose = torch.tensor(scene["view_cell_center"]) + 0.1 * torch.randn(3, generator=g)
+        rot = orc.rotation_yaw(float(seed * 17))
+        st = ref.stages(pose, rot, dirs_all[pix])
+        rows = np.sort(np.random.default_rng(seed).choice(n_rays, n_raw0, replace=False))
+        arrays.update({tag + "/pix": pix.numpy().astype(np.int32), tag + "/pose": pose.numpy(), tag + "/rot": rot.numpy(),
+                       tag + "/raw0_rows": rows.astype(np.int32), tag + "/raw0": st["raw0"][rows], tag + "/asp": st["asp"],
+                       tag + "/rgb": st["rgb"], tag + "/weights": st["weights"]})
+    save("fresh_seeds.npz", **arrays)
+
+
+def train_config_fields():
+    """The attributes B200Inference.args_from_train_config reads, as an initialised reference TrainConfig carries them."""
+    scene = orc.SCENE_PAVILLON
+    cases = []
+    for K, thr in ((8, 0.2), (16, 0.15)):
+        ref = rh.RefRenderer(scene, K=K, thr=thr)
+        f1, view = ref.tc.f_in[1], ref.dataset_info.view
+        fields = {a: getattr(f1, a) for a in ("depth_range", "max_depth", "z_near", "z_far", "n_ray_samples", "useNDC", "w", "h")
+                  if hasattr(f1, a)}
+        cases.append(dict(K=K, thr=thr, f_in_1=dict(fields, z_sampler=dict(threshold=f1.z_sampler.threshold)),
+                          view={a: getattr(view, a) for a in ("view_cell_center", "view_cell_size", "fov", "focal")},
+                          state_dict_keys=[list(m.state_dict()) for m in ref.tc.models]))
+    path = os.path.join(OUT, "train_config_fields.json")
+    with open(path, "w") as f:
+        json.dump(dict(source="reference TrainConfig (FeatureSet.initialize + ModelSelection.getModel, CPU)",
+                       torch_version=torch.__version__, cases=cases), f, indent=1)
+        f.write("\n")
+    print(f"wrote {path}")
+
+
+def shrink_onnx(src, dst, keep=4):
+    """Copies an ONNX model field for field, except that every fp32 initialiser keeps only its leading
+    keep x keep block (dims rewritten to match): the exporter's layout at a few kB."""
+    buf = memoryview(open(src, "rb").read())
+
+    def copy(fn, wt, v):
+        if wt == 0:
+            return _field(fn, 0, v)
+        if wt == 2:
+            return _field(fn, 2, bytes(buf[v[0]:v[1]]))
+        return _enc_varint((fn << 3) | wt) + bytes(buf[v[0]:v[1]])     # fixed-width payload, no length
+
+    def tensor(s, e):
+        fields = list(_fields(buf, s, e))
+        dims = []
+        for fn, wt, v in fields:
+            if fn == 1 and wt == 0:
+                dims.append(v)
+            elif fn == 1:
+                p = v[0]
+                while p < v[1]:
+                    d, p = _varint(buf, p)
+                    dims.append(d)
+        if not any(fn == 2 and v == 1 for fn, _, v in fields):      # not FLOAT: unchanged
+            return bytes(buf[s:e])
+        raw = next(v for fn, _, v in fields if fn == 9)
+        arr = np.frombuffer(buf, dtype="<f4", count=(raw[1] - raw[0]) // 4, offset=raw[0]).reshape(dims)
+        small = np.ascontiguousarray(arr[tuple(slice(0, keep) for _ in dims)])
+        out, dims_done = b"", False
+        for fn, wt, v in fields:
+            if fn == 1:
+                if not dims_done:
+                    out += b"".join(_field(1, 0, d) for d in small.shape)
+                    dims_done = True
+            elif fn == 9:
+                out += _field(9, 2, small.tobytes())
+            else:
+                out += copy(fn, wt, v)
+        return out
+
+    def graph(s, e):
+        return b"".join(_field(5, 2, tensor(*v)) if fn == 5 and wt == 2 else copy(fn, wt, v) for fn, wt, v in _fields(buf, s, e))
+
+    model = b"".join(_field(7, 2, graph(*v)) if fn == 7 and wt == 2 else copy(fn, wt, v) for fn, wt, v in _fields(buf, 0, len(buf)))
+    with open(dst, "wb") as f:
+        f.write(model)
+    print(f"wrote {dst}  ({len(model)} bytes, from {len(buf)})")
+
+
+def shipped_sample():
+    """The viewer's shipped export directory: config.ini and dataset_info.txt verbatim, model{0,1}.onnx shrunk."""
+    src = os.path.join(rh.REF_ROOT, "adanerf_real_time_viewer", "sample")
+    dst = os.path.join(OUT, "viewer_sample")
+    os.makedirs(dst, exist_ok=True)
+    for name in ("config.ini", "dataset_info.txt"):
+        shutil.copyfile(os.path.join(src, name), os.path.join(dst, name))
+    for i in range(2):
+        shrink_onnx(os.path.join(src, f"model{i}.onnx"), os.path.join(dst, f"model{i}.onnx"))
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(8)
@@ -126,7 +249,15 @@ def main():
     stage_case("ndc_k16_t0.15", "pavillon_ndc", orc.SCENE_PAVILLON_NDC, n0, n1, 16, 0.15, 256, 2501, [0.1, -0.05, 0.02],
                orc.rotation_yaw(20.0), True, ndc=True)
     stage2_stress()
+    fresh_seeds()
+    train_config_fields()
+    shipped_sample()
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) > 1:               # e.g. `python oracle/gen_golden.py fresh_seeds`: only the named fixtures
+        torch.set_num_threads(8)
+        for name in sys.argv[1:]:
+            globals()[name]()
+    else:
+        main()

@@ -78,7 +78,7 @@ class _NS:
 
 def _duck_train_config(m, sd0, sd1, K, thr):
     """An object with exactly the attributes B200Inference.from_train_config reads from an initialised reference
-    TrainConfig (tests/test_adapter_config.py pins those names against the live reference on a CPU box)."""
+    TrainConfig (tests/test_adapter_config.py pins those names against the fields of a reference TrainConfig)."""
     sp = m["scene_params"]
     view = _NS(view_cell_center=sp["view_cell_center"], view_cell_size=sp["view_cell_size"], fov=sp["fov"], focal=None)
     f1 = _NS(depth_range=sp["depth_range"], max_depth=sp["max_depth"], z_near=0.001, z_far=1.0, useNDC=False,

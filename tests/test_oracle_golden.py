@@ -1,12 +1,13 @@
 """Pins oracle/adanerf_oracle.py against fixtures produced by the unmodified reference
-(oracle/gen_golden.py), and -- when /root/reference is mounted -- against the live reference."""
+(oracle/gen_golden.py)."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden, case_weights
+from conftest import GOLDEN, load_golden, case_weights
 from oracle import adanerf_oracle as orc
-from oracle import ref_harness as rh
 
 CASES = ["pav_k8_t0.2", "pav_k8_t0.5", "pav_k16_t0.15", "shaped_k8_t0.2", "rand_k8_t0.2", "ndc_k16_t0.15"]
 
@@ -130,26 +131,29 @@ def test_weight_init_is_reproducible():
     assert a1["views_linears.0.weight"].shape == (128, 283)
 
 
-@pytest.mark.skipif(not rh.available(), reason="/root/reference not mounted (GPU box)")
 @pytest.mark.parametrize("seed,K,thr", [(11, 8, 0.2), (12, 4, 0.05), (13, 16, 0.3)])
 def test_live_reference_fresh_seed(seed, K, thr):
+    """The reference initialised from a fresh seed by its own initialisers, then run on 512 random rays with a sampling
+    net shaped for ragged counts (oracle/gen_golden.py: fresh_seeds).  Exact: the initial weights and the sample
+    selection on the reference's own raw0.  To GEMM rounding, which differs between hosts (oneMKL picks its kernels by
+    instruction set): raw0, the sample counts, rgb and the compositing weights."""
+    from oracle.gen_golden import state_dict_digest
+    z = np.load(os.path.join(GOLDEN, "fresh_seeds.npz"), allow_pickle=False)
+    ref = {k.split("/", 1)[1]: z[k] for k in z.files if k.startswith(f"s{seed}/")}
     scene = orc.SCENE_BARBERSHOP
-    ref = rh.RefRenderer(scene, K=K, thr=thr, seed=seed)
     sd0, sd1 = orc.make_weights("rand", seed=seed)
-    assert all(torch.equal(sd0[k], v) for k, v in ref.models[0].state_dict().items())
-    assert all(torch.equal(sd1[k], v) for k, v in ref.models[1].state_dict().items())
-    # shape the sampling net so counts are ragged, then load the same weights into the reference
+    assert [state_dict_digest(sd0), state_dict_digest(sd1)] == ref["init_digest"].tolist()
+    # shape the sampling net so counts are ragged (the reference ran on the same weights)
     sd0["layers.7.weight"] *= 0.15
     sd0["layers.7.bias"] = sd0["layers.7.bias"] * 0.15 - 0.2
-    ref.load_state_dicts(sd0, sd1)
-    g = torch.Generator().manual_seed(seed)
     dirs = torch.from_numpy(orc.generate_ray_directions(800, 800, scene["fov"]).reshape(-1, 3)).float()
-    dirs = dirs[torch.randperm(dirs.shape[0], generator=g)[:512]]
-    pose = torch.tensor(scene["view_cell_center"]) + 0.1 * torch.randn(3, generator=g)
-    rot = orc.rotation_yaw(float(seed * 17))
-    st = ref.stages(pose, rot, dirs)
+    dirs = dirs[torch.from_numpy(ref["pix"]).long()]
+    pose, rot = torch.from_numpy(ref["pose"]), torch.from_numpy(ref["rot"])
+    s2 = orc.stage2_sample(torch.from_numpy(ref["raw0"]), thr, K, scene["depth_range"])
+    np.testing.assert_array_equal((s2["count"].numpy() / K).astype(np.float32), ref["asp"][ref["raw0_rows"]])
     o = orc.render_rays(pose, rot, dirs, sd0, sd1, scene, thr, K, return_stages=True)
-    np.testing.assert_array_equal(o["raw0"].numpy(), st["raw0"])
-    np.testing.assert_array_equal(o["asp"].numpy(), st["asp"])
-    np.testing.assert_array_equal(o["rgb"].numpy(), st["rgb"])
-    np.testing.assert_array_equal(o["weights"].numpy(), st["weights"])
+    np.testing.assert_allclose(o["raw0"].numpy()[ref["raw0_rows"]], ref["raw0"], rtol=0, atol=5e-4)
+    same = o["asp"].numpy() == ref["asp"]
+    assert same.mean() > 0.98
+    np.testing.assert_allclose(o["rgb"].numpy()[same], ref["rgb"][same], rtol=0, atol=2e-4)
+    np.testing.assert_allclose(o["weights"].numpy()[same], ref["weights"][same], rtol=0, atol=2e-4)
